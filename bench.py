@@ -15,6 +15,10 @@ CUDA events on the stream the kernels run on, max over ranks. `e2e` = the same m
 the C ABI one round per call with host buffers: every step uploads that round's event trace,
 runs one round and reads the counters and the convergence count back
 (swim_sim_inject + swim_sim_step_async(1) + swim_sim_observe, one synchronisation per round).
+
+`--dump-outputs DIR` writes, after the timed windows, what the last of them left on the handle (write_outputs) as
+DIR/<name>.npy: the inputs depend on the arguments alone, so two builds run with the same arguments can be compared
+file by file (and the CUDA arm with `--impl reference`).
 """
 import argparse
 import json
@@ -84,6 +88,49 @@ def algorithmic_bytes(cfg_kw, n_nodes, rounds, ctr_delta):
     floor = 7 * D + 16 * B + 4 * F + 8
     msg_side = (8 + 8 * b_bar) * m_bar  # written once (tick) and read once (receive)
     return floor + 2 * msg_side, floor + msg_side, m_bar, b_bar
+
+
+DUMP_NODES = 32768  # rows written by --dump-outputs: a fixed sample of node ids (C3's full state is 0.5 GB per GPU)
+DUMP_SEED = 0xD0
+DUMP_MAX_BYTES = 64 << 20
+
+
+def write_outputs(h, out_dir, n_nodes, rank=0, world=1):
+    """What a caller of the timed path reads back after its last step, as float64 arrays in out_dir/<name>.npy:
+    counters (A.CTR_NAMES order, summed over ranks), mismatches (the convergence count), digest (the 64-bit state digest
+    as [high, low] 32-bit halves), and every state array of A.ARRAY_NAMES — the piggyback records field by field as
+    pb_<field> — at the rows of sample_nodes, DUMP_NODES node ids drawn with a fixed seed. `h` is a Simulator or an
+    Oracle. With world > 1 every rank must call this (it gathers) and rank 0 writes."""
+    nodes = np.sort(np.random.default_rng(DUMP_SEED).choice(n_nodes, size=min(n_nodes, DUMP_NODES), replace=False))
+    own = nodes[(nodes >= h.first) & (nodes < h.first + h.n_local)]
+    part = {}
+    for a in range(A.ARR_COUNT):
+        full = a in A.REPLICATED_ARRAYS  # [N] on every rank; the other arrays hold this rank's rows only
+        x = h.get_array(a).reshape(n_nodes if full else h.n_local, -1)[own if full else own - h.first]
+        if a == A.ARR_PB:
+            for f in ("member", "incarnation", "from", "kind", "ttl"):
+                part["pb_" + f] = x[f]
+        else:
+            part[A.ARRAY_NAMES[a]] = x if x.shape[1] > 1 else x[:, 0]
+    if world > 1:
+        import torch.distributed as dist
+        from swim_b200 import dist as sdist
+        parts = [None] * world
+        dist.all_gather_object(parts, part)
+        part = {k: np.concatenate([p[k] for p in parts]) for k in part}  # ranks own ascending node ranges
+        ctr, mm, dg = sdist.global_sum(h.counters()), sdist.global_sum([h.mismatches()]), sdist.global_digest(h.digest())
+        if rank != 0:
+            return
+    else:
+        ctr, mm, dg = h.counters(), [h.mismatches()], h.digest()
+    out = dict(part, sample_nodes=nodes, counters=ctr, mismatches=mm, digest=[dg >> 32, dg & 0xFFFFFFFF])
+    out = {k: np.asarray(v).astype(np.float64) for k, v in out.items()}
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes (limit {DUMP_MAX_BYTES})")
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in out.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
 
 
 def timed_kernel_name(steps, world):
@@ -274,7 +321,9 @@ def run_reference(args):
     if rank != 0:
         return None
     cfg_kw, nbr, events, n = workload(args.gpus, args.nodes_per_gpu)  # the same N as the CUDA arm at --gpus G (one shard: all on the host)
-    val, dt, threads, _ = cpu_arm(cfg_kw, nbr, events, n, args.steps, args.warmup)
+    val, dt, threads, orc = cpu_arm(cfg_kw, nbr, events, n, args.steps, args.warmup)
+    if args.dump_outputs:
+        write_outputs(orc, args.dump_outputs, n)
     line = {
         "impl": "reference", "metric": "simulated node-rounds/sec", "value": val, "unit": "node-rounds/s",
         "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup, "ms_per_step": dt * 1e3 / args.steps,
@@ -405,6 +454,8 @@ def run_cuda(args):
         barrier()
         ms_w = ev0.elapsed_time(ev1)
         sim.sync()
+        if sim.round != args.warmup + args.steps:
+            raise RuntimeError(f"timed window ended at round {sim.round}, not {args.warmup} + {args.steps}")
         c1, l1 = sim.counters(), sim.launch_count()
         if world > 1:
             t = torch.tensor([ms_w], device=_TENSOR_DEVICE)
@@ -419,6 +470,8 @@ def run_cuda(args):
             else:
                 ctr_delta = c1 - c0
             launches = int(l1 - l0)
+        if args.dump_outputs and w == args.windows - 1:
+            write_outputs(sim, args.dump_outputs, n, rank, world)
     ms = float(np.median(windows))
     log(f"timed windows done: {windows}")
     value = n * args.steps / (ms * 1e-3)
@@ -712,7 +765,7 @@ class StdoutToStderr:
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=448)
+    ap.add_argument("--steps", type=int, default=448, help="rounds in each timed window")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="cuda", choices=["cuda", "reference"])
     ap.add_argument("--nodes-per-gpu", type=int, default=N_PER_GPU)
@@ -724,7 +777,11 @@ def main():
     ap.add_argument("--spinup", type=float, default=0.5, help="seconds of untimed rounds before the first window (GPU clocks)")
     ap.add_argument("--exchange", default=None, choices=[None, "p2p", "nccl"],
                     help="cross-shard exchange: fused peer-memory (default) or staged NCCL all-to-all")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state the last timed window computed to DIR/<name>.npy (float64, a seeded node sample)")
     args = ap.parse_args()
+    if args.steps < 1 or args.windows < 1:
+        ap.error("--steps and --windows must be at least 1")
     if args.warmup < 3:
         args.warmup = 3
     with StdoutToStderr():

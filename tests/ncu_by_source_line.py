@@ -62,7 +62,7 @@ for loc, (ex, st) in sorted(agg.items(), key=lambda x: -x[1][0])[:int(sys.argv[4
 if len(sys.argv) > 6:
     a, b = int(sys.argv[5]), int(sys.argv[6])
     print('--- lines', a, b)
-    srcl = open('/root/repo/swim_b200/csrc/swim_device.cuh').read().splitlines()
+    srcl = src_lines
     for loc, (ex, st) in sorted((x for x in agg.items() if x[0] and x[0][0] == 'swim_device.cuh' and a <= x[0][1] <= b), key=lambda x: x[0][1]):
         if ex > 150000 or st > 100:
             print(f'{loc[1]:5d} exec {ex/16/1000:7.1f}k/round stalls {st:6d} | {srcl[loc[1]-1].strip()[:110]}')

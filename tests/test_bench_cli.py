@@ -24,6 +24,25 @@ def test_reference_arm_prints_one_json_line():
     assert d["config"]["n_nodes"] == 1 << 20 and "workload" in d["config"]
 
 
+def test_reference_arm_dump_outputs_are_bounded_and_repeatable(tmp_path):
+    """--dump-outputs at the full C3 size: float64 files within 64 MB, the same bytes from two runs with the same arguments."""
+    import numpy as np
+    dumps = []
+    for run in ("a", "b"):
+        out = tmp_path / run
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "3", "--warmup", "3",
+                            "--dump-outputs", str(out)], capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stderr[-2000:]
+        dumps.append({f: np.load(out / f) for f in sorted(os.listdir(out))})
+    a, b = dumps
+    assert sorted(a) == sorted(b) and "counters.npy" in a and "nbr.npy" in a
+    assert sum(os.path.getsize(tmp_path / "a" / f) for f in a) <= 64 << 20
+    assert len(a["sample_nodes.npy"]) == 32768 and a["nbr.npy"].shape == (32768, 32)
+    for f in a:
+        assert a[f].dtype == np.float64 and np.array_equal(a[f], b[f]), f
+    assert a["counters.npy"][0] > 0  # pings of 6 rounds
+
+
 def test_reference_arm_uses_all_host_threads_under_torchrun():
     """torchrun exports OMP_NUM_THREADS=1; the CPU arm must still use every core it may."""
     if len(os.sched_getaffinity(0)) < 2:

@@ -57,7 +57,7 @@ def test_cuda_arm_runs_every_leg_on_the_emulator(emulated_bench, steps, xmode, m
     if xmode is not None:
         monkeypatch.setenv("SWIM_XMODE", xmode)
     args = argparse.Namespace(gpus=1, steps=steps, warmup=5, impl="cuda", nodes_per_gpu=8192, converge_limit=160, no_cpu=False,
-                              no_parity=False, no_ring=False, windows=2, spinup=0.0, exchange=None)
+                              no_parity=False, no_ring=False, windows=2, spinup=0.0, exchange=None, dump_outputs=None)
     line = bench.run_cuda(args)
     json.dumps(line)  # serialisable
     assert line["metric"] == "simulated node-rounds/sec" and line["n_gpus"] == 1 and line["steps"] == steps
@@ -77,6 +77,41 @@ def test_cuda_arm_runs_every_leg_on_the_emulator(emulated_bench, steps, xmode, m
     g = line["state_machine_workload"]
     assert g["parity_check"] == "ok" and g["value"] > 0
     assert line["config"]["n_nodes"] == 8192 and "workload" in line["config"]
+
+
+def _check_dump(bench, out_dir, n_nodes, rounds, tmp_path):
+    """What --dump-outputs wrote is the state the oracle reaches after the same rounds of the same workload, file for file."""
+    import numpy as np
+    from oracle.oracle import Oracle
+    from swim_b200.sim import default_config
+    cfg_kw, nbr, events, n = bench.workload(1, n_nodes)
+    orc = Oracle(default_config(**cfg_kw))
+    orc.set_view(nbr)
+    orc.inject(events)
+    orc.step(rounds)
+    want = tmp_path / "oracle_outputs"
+    bench.write_outputs(orc, str(want), n)
+    names = sorted(os.listdir(out_dir))
+    assert names == sorted(os.listdir(want))
+    assert {"counters.npy", "digest.npy", "mismatches.npy", "sample_nodes.npy", "nbr.npy", "pb_member.npy"} <= set(names)
+    for f in names:
+        got = np.load(os.path.join(out_dir, f))
+        assert got.dtype == np.float64 and np.array_equal(got, np.load(want / f)), f
+    assert np.load(want / "counters.npy").tolist() == [float(x) for x in orc.counters()]
+    assert len(np.load(want / "sample_nodes.npy")) == min(n, bench.DUMP_NODES)
+
+
+def test_dump_outputs_on_the_emulator(emulated_bench, tmp_path, monkeypatch):
+    """--dump-outputs: the state of the last timed round (warm-up + steps), sampled when the node set is larger than
+    DUMP_NODES, equals the oracle's."""
+    bench = emulated_bench
+    monkeypatch.setattr(bench, "DUMP_NODES", 1000)
+    out = tmp_path / "outputs"
+    args = argparse.Namespace(gpus=1, steps=12, warmup=5, impl="cuda", nodes_per_gpu=4096, converge_limit=40, no_cpu=True,
+                              no_parity=True, no_ring=True, windows=2, spinup=0.0, exchange=None, dump_outputs=str(out))
+    line = bench.run_cuda(args)
+    assert line["steps"] == 12
+    _check_dump(bench, out, 4096, 5 + 12, tmp_path)
 
 
 # ---------------------------------------------------------------- the sharded flow: ranks as threads of one process
@@ -121,7 +156,7 @@ class _ThreadDist:
 
 
 @pytest.mark.parametrize("world,steps", [(2, 20), (3, 12)])
-def test_sharded_cuda_arm_on_the_emulator(emulated_bench, world, steps, monkeypatch):
+def test_sharded_cuda_arm_on_the_emulator(emulated_bench, world, steps, monkeypatch, tmp_path):
     """bench.py --gpus N with the ranks as threads (each with its own handle on the emulated device, connected through raw
     peer pointers exactly as ranks of one process are on hardware): the collective structure of every leg — load as a
     collective, the spin-up that ends on one decision for all ranks, streams drained before barriers, the end-to-end loop
@@ -158,7 +193,8 @@ def test_sharded_cuda_arm_on_the_emulator(emulated_bench, world, steps, monkeypa
     def rank_main(r):
         fake.tl.rank = r
         args = argparse.Namespace(gpus=world, steps=steps, warmup=5, impl="cuda", nodes_per_gpu=2048, converge_limit=120, no_cpu=True,
-                                  no_parity=False, no_ring=True, windows=2, spinup=0.05, exchange=None)
+                                  no_parity=False, no_ring=True, windows=2, spinup=0.05, exchange=None,
+                                  dump_outputs=str(tmp_path / "outputs"))
         try:
             lines[r] = bench.run_cuda(args)
         except BaseException as e:  # noqa: BLE001
@@ -179,3 +215,4 @@ def test_sharded_cuda_arm_on_the_emulator(emulated_bench, world, steps, monkeypa
     assert line["parity_check"] == "ok", line["parity"]
     assert line["value"] > 0 and line["e2e"]["value"] > 0 and line["e2e"]["api"] == "swim_sim_step_observe"
     assert line["convergence"] is not None and line["state_machine_workload"] is None and line["cpu_baseline"] is None
+    _check_dump(bench, tmp_path / "outputs", 2048 * world, 5 + steps, tmp_path)  # the shards' rows, gathered by rank 0
